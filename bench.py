@@ -2,6 +2,7 @@
 """Benchmark of the SAMBLE hot path on B200 (contract: README of the task / DESIGN.md section 6).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload seg|cls|knn_ds] [--batch B | --global-batch G] [--points N]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...        # the reference's CPU algorithm (oracle port) on host cores
 
@@ -15,6 +16,10 @@ All in eval mode with frozen bin boundaries and topk sampling, on synthetic clou
 `value` = clouds/s with inputs resident in HBM (whole step replayed as one CUDA graph); `e2e` = the same forward fed
 from HOST (pinned) buffers with a host copy of the result, every copy inside the timed region.  The batch is sharded
 by cloud across ranks with no collective on the path.  One JSON line is printed by rank 0.
+`--steps K` is the number of timed steps (graph replays for knn_ds) of every arm.
+--dump-outputs DIR (seg / cls, native): the logits of the last timed step, all ranks' clouds in order, go to
+DIR/logits.npy.  Inputs, weights and the calibration batch are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -48,8 +53,14 @@ def parse():
     ap.add_argument("--cpu-steps", type=int, default=2)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="launch kernel by kernel instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the logits of the last timed step as DIR/logits.npy (float32)")
     a = ap.parse_args()
     a.points = a.points or (1024 if a.workload == "cls" else 2048)
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "native" or a.workload == "knn_ds"):
+        ap.error("--dump-outputs writes the logits of the native seg / cls forward")
     return a
 
 
@@ -148,17 +159,17 @@ def run_reference(args):
     B = per_rank_batch(args, world)
     cores = max(1, len(os.sched_getaffinity(0)))
     if args.workload == "knn_ds":
-        res = {str(N): cpu_knn_ds(N) for N in (8192, 16384)}
+        res = {str(N): cpu_knn_ds(N, reps=args.steps) for N in (8192, 16384)}
         line = {"impl": "reference", "metric": METRICS["knn_ds"], "value": res["8192"]["downsample_token_s"] * 1e6, "unit": "us/batch",
-                "n_gpus": args.gpus, "steps": 1, "warmup": 0, "higher_is_better": False, "scaling": "weak", "vs_baseline": None,
+                "n_gpus": args.gpus, "steps": args.steps, "warmup": 0, "higher_is_better": False, "scaling": "weak", "vs_baseline": None,
                 "dtype": "f32", "data": "synthetic", "config": workload_config(args, world, 1), "results_s_per_call_B1": res,
                 "cpu_baseline": {"value": res["8192"]["downsample_token_s"] * 1e6, "unit": "us/batch", "cores": cores, "kind": "port",
-                                 "sample": "oracle knn (C=3, C=128) and downsample_token at B=1, N=8192 and 16384, one call each"},
+                                 "sample": f"oracle knn (C=3, C=128) and downsample_token at B=1, N=8192 and 16384, {args.steps} calls each"},
                 "e2e": {"value": res["8192"]["downsample_token_s"] * 1e6, "unit": "us/batch", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}
         print(json.dumps(line), flush=True)
         return
-    # a bounded sample of the same workload: the SAME per-GPU batch as the native arm, few steps
-    steps, warmup = max(1, min(args.steps, 3)), 1
+    # the SAME per-GPU batch as the native arm (a CPU step takes seconds at the default size: pass a small --steps)
+    steps, warmup = args.steps, 1
     rate, dt = cpu_reference_rate(args.workload, B, args.points, steps, warmup)
     line = {"impl": "reference", "metric": METRICS[args.workload], "value": rate, "unit": UNIT, "n_gpus": args.gpus, "steps": steps,
             "warmup": warmup, "ms_per_step": dt * 1e3, "higher_is_better": True,
@@ -387,7 +398,7 @@ def run_knn_ds(args, dev, pk, pk_src, flush):
         res = {"B": B}
         for C in (3, 128):
             a = synthetic_features(B, N, C, 3).to(dev)
-            us = graphed_us(lambda: ops.knn(a, a, 32), flush=flush)
+            us = graphed_us(lambda: ops.knn(a, a, 32), reps=args.steps, flush=flush)
             flops = 2.0 * N * N * C * B
             res[f"knn_c{C}"] = {"us_per_batch": us, "algorithmic_tflops": flops / (us * 1e-6) / 1e12,
                                  "bound": "fp32 pipe" if C == 3 else "tensor",
@@ -401,12 +412,30 @@ def run_knn_ds(args, dev, pk, pk_src, flush):
         with torch.no_grad():
             ds(x)
         ds.dynamic_boundaries_enable = False
-        us = graphed_us(lambda: ds(x), flush=flush)
+        us = graphed_us(lambda: ds(x), reps=args.steps, flush=flush)
         fl = ds_flops(N, N // 2) * B
         res["downsample_token"] = {"us_per_batch": us, "algorithmic_tflops": fl / (us * 1e-6) / 1e12, "bound": "tensor",
                                    "frac": fl / (us * 1e-6) / 1e12 / bf16}
         out[str(N)] = res
     return out
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(directory, name, y):
+    """Write y (clouds along dim 0) as <directory>/<name>.npy in float32.  When that would exceed DUMP_BYTES, a fixed
+    seeded sample of whole clouds is written instead and their indices (ascending) go to <name>_clouds.npy (float64)."""
+    import numpy as np
+
+    y = y.float().cpu()
+    os.makedirs(directory, exist_ok=True)
+    if y.numel() * 4 > DUMP_BYTES:
+        keep = (DUMP_BYTES - 1024) // (y[0].numel() * 4 + 8)    # room for both .npy headers and the indices
+        idx = torch.randperm(y.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        y = y[idx]
+        np.save(os.path.join(directory, f"{name}_clouds.npy"), idx.double().numpy())
+    np.save(os.path.join(directory, f"{name}.npy"), y.numpy())
 
 
 def run_native(args):
@@ -438,7 +467,7 @@ def run_native(args):
             sampler.stop_flag = True
             sampler.join()
             line = {"metric": METRICS["knn_ds"], "value": res["8192"]["downsample_token"]["us_per_batch"], "unit": "us/batch", "n_gpus": 1,
-                    "steps": 20, "warmup": 5, "higher_is_better": False, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
+                    "steps": args.steps, "warmup": 5, "higher_is_better": False, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
                     "data": "synthetic", "config": workload_config(args, 1, res["8192"]["B"]), "clocks": sampler.result(),
                     "results": res, "gpu_launches": int(lib.samble_launch_count())}
             if not args.no_cpu_baseline:
@@ -507,8 +536,10 @@ def run_native(args):
             run = GraphedForward(model, *ins)              # whole step = one graph launch
             pipe = HostPipeline(run)       # the serving loop a host-resident caller uses: D2H of step i overlaps step i+1
 
+        last = {}
+
         def step_resident():
-            run(*ins)
+            last["y"] = run(*ins)
 
         def step_e2e():
             # every timed step contains: H2D of its inputs, the forward, and the wait for the PREVIOUS step's D2H (which
@@ -525,6 +556,8 @@ def run_native(args):
         sampler = ClockSampler(local)
         sampler.start()
         ms, per_rank, launches = timed(step_resident, args.steps)
+        # (the graph's output buffer is overwritten by the e2e steps below)
+        y_last = last["y"].clone() if args.dump_outputs else None
         for _ in range(2):
             step_e2e()
         ms_e2e, per_rank_e2e, _ = timed(step_e2e, args.steps, tail_fn=(pipe.wait_all if pipe is not None else None))
@@ -559,6 +592,13 @@ def run_native(args):
 
     value = B * world * args.steps / (ms / 1e3)
     e2e_value = B * world * args.steps / (ms_e2e / 1e3)
+    if args.dump_outputs:
+        ys = [y_last]
+        if world > 1:
+            ys = [torch.empty_like(y_last) for _ in range(world)]
+            dist.all_gather(ys, y_last)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, "logits", torch.cat(ys))
     if rank != 0:
         if world > 1:
             dist.destroy_process_group()

@@ -22,8 +22,8 @@ Pinning status
 --------------
 The reference ships NO tests, golden vectors or known-answer files (SURVEY 4), so
 nothing upstream pins this oracle.  It is pinned instead against outputs of the
-reference itself, run in the authoring container by tests/golden/make_golden.py
-(committed fixtures in tests/golden/*.npz) and, when /root/reference is present,
+reference itself, run by tests/golden/make_golden.py (committed fixtures in
+tests/golden/*.npz) and, when SAMBLE_REFERENCE names a checkout of the reference,
 live in tests/test_oracle_vs_reference.py.
 """
 from __future__ import annotations

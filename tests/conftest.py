@@ -10,14 +10,14 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu on the GPU box)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (authoring container only)")
+    config.addinivalue_line("markers", "needs_reference: needs a checkout of upstream SAMBLE named by SAMBLE_REFERENCE")
 
 
 def pytest_collection_modifyitems(config, items):
     from tests.golden import ref_loader
 
     have_ref = ref_loader.available()
-    skip_ref = pytest.mark.skip(reason="/root/reference not present on this box")
+    skip_ref = pytest.mark.skip(reason="SAMBLE_REFERENCE does not name a checkout of upstream SAMBLE")
     for item in items:
         if "needs_reference" in item.keywords and not have_ref:
             item.add_marker(skip_ref)

@@ -1,10 +1,10 @@
-"""Mint golden vectors from the UNMODIFIED reference (authoring container only).
+"""Mint golden vectors from the UNMODIFIED reference.
 
-    python tests/golden/make_golden.py
+    SAMBLE_REFERENCE=<checkout of upstream SAMBLE> python tests/golden/make_golden.py
 
 The reference ships no tests or known-answer files (SURVEY 4), so the fixtures
 that pin the oracle are outputs of the reference itself, imported from
-/root/reference and run on CPU in eval()/no_grad with
+the SAMBLE_REFERENCE checkout and run on CPU in eval()/no_grad with
   * inputs from samble_b200.testing.synthetic_clouds / synthetic_features (seeded),
   * weights from samble_b200.testing.fill_state_dict_ (a pure function of the entry
     name and a seed, so no weights need to be stored),

@@ -544,9 +544,8 @@ def test_checkpoint_and_eval_harness(tmp_path):
 @pytest.mark.parametrize("which", ["seg", "cls"])
 def test_unmodified_reference_wiring_with_the_patch_installed(which):
     """The drop-in claim end to end: the reference's OWN models/seg_model.py / cls_model.py (unmodified, imported from
-    SAMBLE_REFERENCE or /root/reference) with samble_b200.patch installed, against the wiring mirror the other tests use.
-    Needs the reference checkout next to a GPU, which the build container (no GPU) and the GPU box (no reference) never
-    offer together: it runs wherever a maintainer has both, and is skipped otherwise."""
+    the checkout named by SAMBLE_REFERENCE) with samble_b200.patch installed, against the wiring mirror the other tests
+    use.  Needs a reference checkout next to a GPU: it runs wherever a maintainer has both, and is skipped otherwise."""
     from samble_b200 import patch
     from tests.golden import ref_loader as R
 

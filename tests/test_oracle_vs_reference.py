@@ -1,5 +1,6 @@
 """Live pin of the oracle (and of our config / state_dict mirrors) against the UNMODIFIED reference.
-Runs only where /root/reference exists (the authoring container); skipped on the GPU box."""
+Runs only where SAMBLE_REFERENCE names a checkout of upstream SAMBLE; skipped otherwise (tests/test_oracle_golden.py
+keeps the oracle pinned to the reference's stored outputs)."""
 import pytest
 import torch
 

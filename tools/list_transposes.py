@@ -1,5 +1,5 @@
-import sys, torch, traceback, collections
-sys.path.insert(0, "/root/repo")
+import os, sys, torch, traceback, collections
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from samble_b200 import models, ops
 from samble_b200.config import seg_config
 from samble_b200.testing import fill_state_dict_, synthetic_clouds

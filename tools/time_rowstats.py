@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from samble_b200 import ops
 B, N, D = 16, 2048, 128
 qkv = torch.randn(B, N, 3 * D, device="cuda")
