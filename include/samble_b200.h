@@ -372,9 +372,10 @@ int samble_sampling_probabilities(const float* score, const uint8_t* mask, int B
 /* utils/ops.py:174-236 dynamic bin boundaries, the two steps around the rank average (:191-199):
  * samble_quantile_pick: cut[j-1] = sorted_desc[int(j / nb * n)], j = 1..nb-1 (:182-189);
  * samble_boundary_ema: cut = cut_sum / world, blended into upper[1:] / lower[:-1] (nb floats each, +-inf sentinels kept or
- * created) with the momentum factor when has_old (:201-233). */
+ * created) with the momentum factor when has_old (:201-233), rounded as ATen rounds these statements on CUDA: momentum is
+ * the Python float (double) the reference multiplies by, and 1 - momentum is formed in double before rounding to fp32. */
 int samble_quantile_pick(const float* sorted_desc, long long n, int nb, float* cut, samble_stream_t stream);
-int samble_boundary_ema(const float* cut_sum, int world, float momentum, int has_old, int nb, float* upper, float* lower,
+int samble_boundary_ema(const float* cut_sum, int world, double momentum, int has_old, int nb, float* upper, float* lower,
                         samble_stream_t stream);
 
 /* ------------------------------------------------------------- UpSample ---------

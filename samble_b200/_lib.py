@@ -82,7 +82,7 @@ PROTOTYPES: Dict[str, Tuple[object, tuple]] = {
     "samble_ds_sample": (_i, (_p, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p, _p, _p, _p)),
     "samble_sampling_probabilities": (_i, (_p, _p, _i, _i, _i, _i, _f, _f, _p, _p)),
     "samble_quantile_pick": (_i, (_p, _ll, _i, _p, _p)),
-    "samble_boundary_ema": (_i, (_p, _i, _f, _i, _i, _p, _p, _p)),
+    "samble_boundary_ema": (_i, (_p, _i, C.c_double, _i, _i, _p, _p, _p)),
     "samble_interpolate3_workspace_bytes": (_sz, (_i, _i, _i)),
     "samble_interpolate3": (_i, (_p, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p, _sz, _p)),
     "samble_interpolate3_search": (_i, (_p, _p, _i, _i, _i, _p, _p, _p, _sz, _p)),

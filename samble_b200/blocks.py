@@ -244,9 +244,16 @@ class DownSampleToken(nn.Module):
     idx_mode sparse_col_sqr, mean_relu, res off, sample_mode 'topk'.
 
     Pipeline (no N x N tensor is ever written):
-      [q|k|v] projection (cuBLAS) -> feature kNN (knn.cu) -> row softmax statistics (downsample.cu)
-      -> edge-only column score -> z-score / bins / k per bin / per-bin top-k (sampler.cu)
-      -> attention rows of the M selected points x V (cuBLAS on an M x (N+nb) slab).
+      [q|k|v] projection -> feature kNN (knn.cu) -> row softmax statistics -> edge-only column score (downsample.cu)
+      -> z-score / bins / k per bin / per-bin top-k (sampler.cu) -> attention rows of the M selected points x V.
+
+    Two branches compute the projection, the row statistics and the selected rows (_forward_native):
+      exact  (C <= 128, C % 32 == 0, D == C; DS_EXACT): exact-product GEMM for [q|k|v] and q k^T (xgemm.cu), the rows
+             as one flash-style kernel over the N + nb keys (ds_attend.cu);
+      3xTF32 (every other width, or DS_EXACT = False): tensor-core projection (linear_tc.cu), row statistics on the fast
+             tensor-core kernel when N % 128 == 0 (else ds_rowstats_tc.cu / the FFMA kernel of downsample.cu), the
+             selected rows gathered by ds_select_rows and multiplied by two per-cloud GEMMs (cloud_matmul) when
+             M % 128 == 0 and N <= 4096, else by ATen matmuls on the (B,M,N) slab.
     """
 
     def __init__(self, config_ds, layer):
@@ -352,7 +359,8 @@ class DownSampleToken(nn.Module):
             [self.q_conv.weight, self.k_conv.weight, self.v_conv.weight], dim=0).view(3 * C, C).contiguous())
         # The two contractions that decide the sampled indices run on the exact-product tensor-core GEMM (csrc/xgemm.cu):
         # fp32-class accuracy independent of accumulation order (the 3xTF32 kernels' logit error is exponentiated here).
-        exact = DS_EXACT and C <= 128 and C % 4 == 0 and D == C
+        # The projection's per-cloud max|q|, |k|, |v| come out of the GEMM in groups of C columns, whole 32-column tiles.
+        exact = DS_EXACT and C <= 128 and C % 32 == 0 and D == C
         join_idx = ops.fork(lambda: ops.knn_indices(x, self.K, ordered=False))                # neighbor_mask's kNN (:301), concurrent
         if exact:
             x_rows = ops.rows_of(x)                                            # (B,N,C)
@@ -442,7 +450,10 @@ class UpSampleInterpolation(nn.Module):
     def forward(self, pcd_up, pcd_down, pcd_up_xyz):
         (points_select, idx_select, points_select_xyz), (points_drop, idx_drop) = pcd_down
         slow = differentiable(self, pcd_up, points_select, pcd_up_xyz, points_select_xyz)
-        if not slow and self.distance_type == "xyz" and self.K == 3 and points_select.shape[1] % 4 == 0:
+        # the row kernels (csrc/upsample.cu) read and write 16-byte chunks: the feature width and the column offset of the
+        # interpolated half in [pcd_up | interpolated] must be multiples of 4 floats
+        rows = self.conv[0].out_channels % 4 == 0 and pcd_up.shape[1] % 4 == 0
+        if not slow and self.distance_type == "xyz" and self.K == 3 and rows:
             # point-major throughout: [pcd_up | interpolated] is assembled as rows (the interpolation writes its half in
             # place), res_conv reads it as a GEMM operand, the result is handed on as a (B,C,N) view of rows
             B, C, N = pcd_up.shape

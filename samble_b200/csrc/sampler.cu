@@ -300,13 +300,16 @@ __global__ void quantile_pick_kernel(const float* __restrict__ sorted_desc, long
 }
 // ... and, after the (nb-1)-float all-reduce, average over ranks and blend into the [upper, lower] pair in place
 // (or create it with the +-inf sentinels when there is no previous pair): one launch instead of ~10 element-wise ones.
-__global__ void boundary_ema_kernel(const float* __restrict__ cut_sum, float inv_world, float momentum, int has_old, int nb,
-                                    float* __restrict__ upper, float* __restrict__ lower) {
+// The roundings are ATen's on CUDA for `cut / world` and `upper * m + (1 - m) * cut` (utils/ops.py:198-213): a tensor divided by
+// a Python scalar is multiplied by the fp32 reciprocal, each scalar reaches the kernel rounded to fp32 from the Python
+// double (so 1 - m is fp32(1 - m), not 1.f - fp32(m)), and every product / sum is rounded on its own (no FMA).
+__global__ void boundary_ema_kernel(const float* __restrict__ cut_sum, float inv_world, float momentum, float one_minus_momentum,
+                                    int has_old, int nb, float* __restrict__ upper, float* __restrict__ lower) {
   const int j = threadIdx.x;                              // cut index 0 .. nb-2
   if (j == 0) upper[0] = INFINITY, lower[nb - 1] = -INFINITY;
   if (j < nb - 1) {
-    float c = cut_sum[j] * inv_world;
-    if (has_old) c = upper[j + 1] * momentum + (1.f - momentum) * c;
+    float c = __fmul_rn(cut_sum[j], inv_world);
+    if (has_old) c = __fadd_rn(__fmul_rn(upper[j + 1], momentum), __fmul_rn(one_minus_momentum, c));
     upper[j + 1] = c;
     lower[j] = c;
   }
@@ -402,12 +405,13 @@ extern "C" int samble_quantile_pick(const float* sorted_desc, long long n, int n
   return SAMBLE_OK;
 }
 
-extern "C" int samble_boundary_ema(const float* cut_sum, int world, float momentum, int has_old, int nb, float* upper, float* lower,
+extern "C" int samble_boundary_ema(const float* cut_sum, int world, double momentum, int has_old, int nb, float* upper, float* lower,
                                    samble_stream_t stream) {
   SAMBLE_REQUIRE(cut_sum && upper && lower && world > 0 && nb > 1 && nb <= kMaxBins, "samble_boundary_ema: bad arguments");
   cudaStream_t st = (cudaStream_t)stream;
   SAMBLE_PRE(st);
-  boundary_ema_kernel<<<1, 32, 0, st>>>(cut_sum, 1.f / (float)world, momentum, has_old, nb, upper, lower);
+  boundary_ema_kernel<<<1, 32, 0, st>>>(cut_sum, 1.f / (float)world, (float)momentum, (float)(1.0 - momentum), has_old, nb, upper,
+                                        lower);
   SAMBLE_LAUNCHED("boundary_ema_kernel");
   return SAMBLE_OK;
 }

@@ -18,8 +18,8 @@ from oracle import samble_oracle as O
 from samble_b200 import blocks, models, ops
 from samble_b200.config import cls_config, seg_config
 from oracle import harness
-from samble_b200.testing import (ds_parity, ds_scores_fp64, fill_state_dict_, knn_parity, sampled_index_parity, synthetic_clouds,
-                                 synthetic_features)
+from samble_b200.testing import (amp_excusing_knn_ties, fill_state_dict_, judge_against_reference_scores, sampled_index_parity,
+                                 synthetic_clouds, synthetic_features)
 from tests.golden import make_golden as G
 
 pytestmark = pytest.mark.gpu
@@ -134,48 +134,6 @@ def test_ds_sample_vs_oracle(B, N, nb, M):
 # ---------------------------------------------------------------- blocks
 
 
-def _amp_excusing_knn_ties(x, sd, pre, cheap=False):
-    """(fp64 scores, amplification) for ds_parity; columns whose in-edge set differs between the native kNN and the
-    oracle's (an fp32 near-tie of two distances, adjudicated by the kNN tests) get an unbounded tolerance: one neighbour
-    more or less changes such a score by ~3 % (score = colsum / indeg^2), which says nothing about the scoring kernels."""
-    C = x.shape[1]
-    mine = ops.knn_indices(cu(x), 32).cpu().long()
-    _, theirs = O.knn(x.transpose(1, 2), x.transpose(1, 2), 32)
-    if cheap:             # large clouds: skip the fp64 N x N pass, take a typical amplification for sharpened logits
-        s64, amp = None, torch.full((x.shape[0], x.shape[2]), 100.0, dtype=torch.float64)
-    else:
-        s64, amp = ds_scores_fp64(x, sd[pre + "q_conv.weight"].view(C, C), sd[pre + "k_conv.weight"].view(C, C), sd[pre + "bin_tokens"][0], mine)
-    B, N = amp.shape
-    a = torch.zeros(B, N, N, dtype=torch.bool).scatter_(2, mine, True)
-    b = torch.zeros(B, N, N, dtype=torch.bool).scatter_(2, theirs, True)
-    touched = (a != b).any(dim=1)                                   # (B,N) columns
-    return s64, torch.where(touched, torch.full_like(amp, 1e15), amp), touched
-
-
-def _judge_against_reference_scores(ds, idx, x_ds, ref_score, ref_idx, ref_k, ref_x_ds, amp):
-    """One DownSampleToken decision against the REFERENCE's own fp32 scores of the same input (golden file or oracle):
-    every bin membership and every per-bin choice must be the one those scores dictate, except where they cannot
-    decide: a z-score within fp32 rounding of a cut (a freshly calibrated cut IS some point's z), keys closer than one
-    rounding of score + 1e-8, or scores closer than the reference's OWN fp32 error (16 roundings x the softmax's
-    amplification `amp`, testing.ds_scores_fp64; measured 1e-5 for the reference, 3e-6 for the native kernels).
-    Rows of x_ds are compared wherever the same point was chosen, unconditionally."""
-    cuts = ds.bin_boundaries[0].reshape(-1)[1:].cpu()
-    rep = ds_parity(ref_score[:, 0].double(), amp, cuts, idx, ds.bin_points_mask, ds.k_point_to_choose, ulps=16.0)
-    print(rep)
-    assert rep["unexplained_bin_flips"] == 0 and rep["unexplained_topk_swaps"] == 0, rep
-    assert rep["chosen_outside_bin"] == 0 and rep["duplicate_rows"] == 0, rep
-    assert rep["distinct_flipped_z_per_cloud"] <= 8, rep     # only points (nearly) tied with a cut flip -- as whole tie groups
-    k_mine = ds.k_point_to_choose.cpu().long()
-    assert int((k_mine - ref_k.long()).abs().max()) <= 1 and bool((k_mine.sum(1) == idx.shape[-1]).all())
-    same = idx.cpu() == ref_idx                              # (B,1,M)
-    key = ref_score + 1e-8                                   # the reference's fp32 sort key: equal keys are ordered arbitrarily
-    tie = key.gather(2, idx.cpu()) == key.gather(2, ref_idx)
-    assert float((same | tie).float().mean()) >= 0.98, float((same | tie).float().mean())
-    ok = ((x_ds.cpu().double() - ref_x_ds.double()).abs() <= 2e-4 + 2e-4 * ref_x_ds.double().abs())       # (B,C,M)
-    assert bool(ok[same.expand_as(ok)].all()), "x_ds rows of identically chosen points differ"
-
-
-
 def _sd(N, M=None, seed=5, sharpen=4.0):
     cfg = seg_config(M=M or (N // 2, N // 4))
     m = models.ShapeNetModel(cfg)
@@ -200,10 +158,10 @@ def test_blocks_golden():
             torch.testing.assert_close(ds.bin_boundaries[0].cpu(), torch.from_numpy(gold[f"ds0.{tag}.upper"]), rtol=1e-5, atol=1e-6)
             gscore = torch.from_numpy(gold[f"ds0.{tag}.score"])
             torch.testing.assert_close(ds.bin_weights_beforerelu.cpu(), torch.from_numpy(gold[f"ds0.{tag}.w"]), atol=1e-5, rtol=1e-4)
-            _, amp, touched = _amp_excusing_knn_ties(x128, sd, "block.downsample_list.0.")
+            _, amp, touched = amp_excusing_knn_ties(x128, sd, "block.downsample_list.0.")
             ok = (ds.attention_point_score.cpu()[:, 0] - gscore[:, 0]).abs() <= 5e-5 * gscore[:, 0].abs() + 1e-30
             assert bool((ok | touched).all()) and int(touched.sum()) <= 8, (int((~ok).sum()), int(touched.sum()))
-            _judge_against_reference_scores(ds, idx, x_ds, gscore, torch.from_numpy(gold[f"ds0.{tag}.idx"]),
+            judge_against_reference_scores(ds, idx, x_ds, gscore, torch.from_numpy(gold[f"ds0.{tag}.idx"]),
                                             torch.from_numpy(gold[f"ds0.{tag}.k"]), torch.from_numpy(gold[f"ds0.{tag}.x_ds"]), amp)
             ds.dynamic_boundaries_enable = False
         xyz_up, xyz_dn = synthetic_features(2, 3, N, 64), synthetic_features(2, 3, N // 2, 65)
@@ -231,11 +189,11 @@ def test_blocks_vs_oracle(N):
             assert tuple(ds.bin_points_mask.shape) == tuple(ref["mask"].shape) and ds.bin_points_mask.dtype == torch.bool
             assert close_frac(ds.attention_bins_beforesoftmax, ref["token_logits"]) == 1.0
             # the exact-product GEMM (csrc/xgemm.cu) puts the native score within a few fp32 roundings of the fp64 value
-            s64, amp, touched = _amp_excusing_knn_ties(x128, sd, pre)
+            s64, amp, touched = amp_excusing_knn_ties(x128, sd, pre)
             big = s64 > 1e-30                                 # (below that the fp32 probabilities underflow)
             rel = (ds.attention_point_score.cpu().double()[:, 0] - s64).abs()[big] / s64[big]
             assert float(rel.max()) <= 2e-5, float(rel.max())
-            _judge_against_reference_scores(ds, idx, x_ds, ref["score"], ref["idx"], ref["k"], ref["x_ds"], amp)
+            judge_against_reference_scores(ds, idx, x_ds, ref["score"], ref["idx"], ref["k"], ref["x_ds"], amp)
             ds.dynamic_boundaries_enable, st.dynamic = False, False
         M = N // 2
         xyz_up, xyz_dn, dn = synthetic_features(B, 3, N, 74), synthetic_features(B, 3, M, 75), synthetic_features(B, 128, M, 76)
@@ -260,10 +218,10 @@ def test_downsample_block_large_clouds(N):
             (x_ds, idx), _ = ds(cu(x))
             ref = O.downsample_token(sd, pre, x, N // 2, 32, 4, st)
             torch.testing.assert_close(ds.bin_boundaries[0].cpu(), ref["boundaries"][0], rtol=1e-5, atol=1e-6)
-            _, amp, touched = _amp_excusing_knn_ties(x, sd, pre, cheap=True)
+            _, amp, touched = amp_excusing_knn_ties(x, sd, pre, cheap=True)
             ok = (ds.attention_point_score.cpu()[:, 0] - ref["score"][:, 0]).abs() <= 2e-4 * ref["score"][:, 0].abs() + 1e-30
             assert bool((ok | touched).all()), int((~(ok | touched)).sum())
-            _judge_against_reference_scores(ds, idx, x_ds, ref["score"], ref["idx"], ref["k"], ref["x_ds"], amp)
+            judge_against_reference_scores(ds, idx, x_ds, ref["score"], ref["idx"], ref["k"], ref["x_ds"], amp)
             ds.dynamic_boundaries_enable, st.dynamic = False, False
 
 
@@ -479,13 +437,18 @@ def test_host_pipeline_returns_the_graph_results_in_order():
         assert torch.equal(a, b)
 
 
-@pytest.mark.parametrize("B,N,M,nb,sharp", [(2, 2048, 1024, 4, 4.0), (3, 1024, 512, 6, 2.0), (1, 1000, 300, 4, 4.0), (1, 8192, 4096, 4, 8.0),
-                                            (2, 256, 128, 4, 1.0)])
-def test_ds_attend_rows_vs_fp64(B, N, M, nb, sharp):
+ATTEND_CASES = [(2, 2048, 1024, 4, 4.0, 128), (3, 1024, 512, 6, 2.0, 128), (1, 1000, 300, 4, 4.0, 128), (1, 8192, 4096, 4, 8.0, 128),
+                (2, 256, 128, 4, 1.0, 128), (2, 1024, 512, 8, 4.0, 32), (2, 1000, 300, 8, 4.0, 64), (2, 2048, 1024, 8, 4.0, 96)]
+
+
+@pytest.mark.parametrize("B,N,M,nb,sharp,D", ATTEND_CASES,
+                         ids=["-".join(map(str, c[:5])) + ("" if c[5] == 128 else f"-D{c[5]}") for c in ATTEND_CASES])
+def test_ds_attend_rows_vs_fp64(B, N, M, nb, sharp, D):
     """The flash-style selected-row attention (csrc/ds_attend.cu) against the literal statement of
     models/downsample.py:242-252 in fp64: softmax rows of the selected points over the N point and nb token columns, times
-    [v ; v_tok].  No (B,M,N) tensor on the device side."""
-    D = C = 128
+    [v ; v_tok].  No (B,M,N) tensor on the device side.  D = C below 128 are the widths DownSampleToken's exact path takes
+    for narrower layers (C % 32 == 0)."""
+    C = D
     g = torch.Generator().manual_seed(N + M)
     q = (torch.randn(B, N, D, generator=g) * sharp)
     k = torch.randn(B, N, D, generator=g)
@@ -503,8 +466,39 @@ def test_ds_attend_rows_vs_fp64(B, N, M, nb, sharp):
     amap = torch.softmax(logits, -1).gather(1, idx.unsqueeze(-1).expand(-1, -1, N + nb))          # (B,M,N+nb)
     ref = amap @ torch.cat([v.double(), v_tok.double().unsqueeze(0).expand(B, -1, -1)], 1)
     err = (out.cpu().double() - ref).abs()
-    print(f"ds_attend_rows B={B} N={N} M={M}: max abs err {err.max():.2e} on values of magnitude {ref.abs().max():.1f}")
+    print(f"ds_attend_rows B={B} N={N} M={M} D={D}: max abs err {err.max():.2e} on values of magnitude {ref.abs().max():.1f}")
     assert bool((err <= 5e-5 + 1e-4 * ref.abs()).all()), float(err.max())
+
+
+@pytest.mark.parametrize("B,N,M,nb,D,C,sliced", [(2, 1024, 512, 4, 64, 128, False), (1, 1000, 301, 1, 128, 128, True),
+                                                 (2, 777, 301, 8, 48, 48, True), (3, 512, 8, 6, 256, 256, False)])
+def test_ds_select_rows_vs_fp64(B, N, M, nb, D, C, sliced):
+    """samble_ds_select_rows (the gather in front of DownSampleToken's 3xTF32 row GEMMs) against fp64: q_sel, m_sel and
+    s_sel are the gathered values exactly; tok_mix is sum_t exp(tok - m) / s * v_tok[t], the token columns' share of
+    models/downsample.py:242-252.  M = 301 leaves the kernel's last block of 8 rows partly empty; `sliced` passes q as a
+    column slice of a (B,N,3C) buffer, as the block does."""
+    g = torch.Generator().manual_seed(N + M + D)
+    q = torch.randn(B, N, D, generator=g) * 2
+    rowmax = torch.randn(B, N, generator=g) + 3
+    rowsum = torch.rand(B, N, generator=g) * 10 + 1
+    tok = torch.randn(B, N, nb, generator=g)
+    v_tok = torch.randn(nb, C, generator=g)
+    idx = torch.stack([torch.randperm(N, generator=g)[:M] for _ in range(B)])
+    if sliced:
+        buf = torch.randn(B, N, 3 * C, generator=g)
+        buf[..., :D] = q
+        qg = cu(buf)[..., :D]
+    else:
+        qg = cu(q)
+    q_sel, m_sel, s_sel, tok_mix = ops.ds_select_rows(qg, cu(rowmax), cu(rowsum), cu(tok), cu(v_tok), cu(idx))
+    gat = lambda t: torch.gather(t, 1, idx.view(B, M, *([1] * (t.dim() - 2))).expand(-1, -1, *t.shape[2:]))
+    assert torch.equal(q_sel.cpu(), gat(q))
+    assert torch.equal(m_sel.cpu(), gat(rowmax)) and torch.equal(s_sel.cpu(), gat(rowsum))
+    p = torch.exp(gat(tok).double() - gat(rowmax).double().unsqueeze(-1)) / gat(rowsum).double().unsqueeze(-1)     # (B,M,nb)
+    ref = p @ v_tok.double()
+    err = (tok_mix.cpu().double() - ref).abs()
+    print(f"ds_select_rows tok_mix: max abs err {err.max():.2e} on values of magnitude {ref.abs().max():.2e}")
+    assert bool((err <= 1e-6 + 1e-5 * ref.abs()).all()), float(err.max())
 
 
 def test_checkpoint_and_eval_harness(tmp_path):

@@ -468,3 +468,151 @@ def test_index_points_copy_engine_vs_thread_copy(B, N, C, M, K):
                 assert torch.equal(ops.index_points(cu(pts), cu(idx).to(dt)).cpu(), ref), (mode, dt)
         finally:
             L.lib().samble_set_gather_mode(0)
+
+
+# ---------------------------------------------------------------- 3-NN interpolation: the three entry points
+
+
+def _interp_clouds(B, N, M, C, seed):
+    """an up cloud and a selected cloud of different offset and scale (the search normalises both by the UP cloud's
+    statistics), features (B,C,M)"""
+    g = torch.Generator().manual_seed(seed)
+    up = (torch.rand(B, 3, N, generator=g) * 2 - 1) * 0.7 + torch.tensor([0.5, -1.0, 2.0]).view(1, 3, 1)
+    sel = (torch.rand(B, 3, M, generator=g) * 2 - 1) * 0.9 + torch.tensor([0.4, -0.8, 2.1]).view(1, 3, 1)
+    return up, sel, torch.randn(B, C, M, generator=g)
+
+
+def _interp_all(up, sel, feat, pad=8):
+    """interpolate3 (channel-major), interpolate3_rows and interpolate3_search + interpolate3_gather_rows, the two row
+    forms writing into column slices of NaN-filled (B,N,C+pad) buffers -> (out (B,N,C) x3, idx int64, dist, nn_w, bufs)"""
+    B, C, N = up.shape[0], feat.shape[1], up.shape[2]
+    feat_rows = cu(feat.transpose(1, 2).contiguous())
+    out3, idx3, d3 = ops.interpolate3(cu(up), cu(sel), cu(feat), want_idx=True)
+    bufs = [torch.full((B, N, C + pad), float("nan"), device=DEV) for _ in range(2)]
+    ops.interpolate3_rows(cu(up), cu(sel), feat_rows, bufs[0][..., 4:4 + C])
+    nn_idx, nn_w = ops.interpolate3_search(cu(up), cu(sel))
+    ops.interpolate3_gather_rows(nn_idx, nn_w, feat_rows, bufs[1][..., 4:4 + C])
+    assert torch.equal(nn_idx.long(), idx3)
+    for buf in bufs:
+        assert bool(buf[..., :4].isnan().all()) and bool(buf[..., 4 + C:].isnan().all()), "wrote outside its columns"
+    return (out3.transpose(1, 2), bufs[0][..., 4:4 + C], bufs[1][..., 4:4 + C]), idx3, d3, nn_w
+
+
+@pytest.mark.parametrize("M", [3, 2047, 2048, 2049, 4100])
+@pytest.mark.parametrize("N", [1, 33, 5000])
+@pytest.mark.parametrize("C", [4, 20, 132])
+def test_interpolate3_entry_points_vs_fp64(M, N, C):
+    """models/upsample.py:194-212 through its three native entry points.  The per-element arithmetic of the channel-major
+    kernel and the row kernel is the same (csrc/upsample.cu), so all three give the same bits; the 3-NN sets match the
+    oracle's up to fp32 near-ties (knn_parity), and the output equals the fp64 weighted sum over the native neighbours
+    and distances.  M = 2048 / 2049 / 4100 cross the search's 2048-candidate shared-memory chunks."""
+    B = 2
+    up, sel, feat = _interp_clouds(B, N, M, C, seed=M + N + C)
+    outs, idx, dist, nn_w = _interp_all(up, sel, feat)
+    assert torch.equal(outs[0], outs[1]) and torch.equal(outs[0], outs[2])
+    idx = idx.cpu()
+    assert int(idx.min()) >= 0 and int(idx.max()) < M
+    assert bool((idx[..., 0] != idx[..., 1]).all() & (idx[..., 1] != idx[..., 2]).all() & (idx[..., 0] != idx[..., 2]).all())
+    if N == 1:
+        # the reference normalises by the unbiased std of the up cloud, undefined for one point (its distances are NaN);
+        # the native search then sees every candidate at distance 0 and takes the lowest indices -- finite, in range
+        assert bool(torch.isfinite(outs[0]).all())
+        return
+    _, idx_r, _ = O.select_neighbors_interpolate(up, sel, feat, 3)
+    rep = knn_parity(idx, idx_r, up.transpose(1, 2), sel.transpose(1, 2))
+    assert rep["unexplained_rows"] == 0 and rep["exact_rate"] >= 0.99, rep
+    # distances in the reference's normalised units (centred and scaled by the up cloud's statistics, utils/ops.py:23-35)
+    up64, sel64 = up.double().transpose(1, 2), sel.double().transpose(1, 2)
+    sigma = up64.std(dim=1, keepdim=True).mean(dim=2, keepdim=True)
+    d64 = torch.linalg.norm(up64.unsqueeze(2) - sel64.gather(1, idx.view(B, -1, 1).expand(-1, -1, 3)).view(B, N, 3, 3), dim=-1)
+    d64 = d64 / sigma
+    assert float((dist.cpu().double() - d64).abs().max()) < 5e-3              # GEMM-form cancellation, as test_knn_vs_oracle
+    w = 1.0 / (dist.cpu().double() + 1e-8)
+    w = w / w.sum(-1, keepdim=True)
+    torch.testing.assert_close(nn_w.cpu().double(), w, atol=1e-6, rtol=1e-6)
+    nbr = feat.double().transpose(1, 2).gather(1, idx.view(B, -1, 1).expand(-1, -1, C)).view(B, N, 3, C)
+    ref = (nbr * w.unsqueeze(-1)).sum(2)                                        # (B,N,C)
+    torch.testing.assert_close(outs[0].cpu().double(), ref, atol=2e-5, rtol=1e-4)
+
+
+def test_interpolate3_coincident_and_duplicate_points():
+    B, N, M, C = 1, 300, 64, 8
+    up, sel, feat = _interp_clouds(B, N, M, C, seed=7)
+    # (1) two selected points at identical coordinates: a tie broken towards the lower index in every entry point
+    sel[:, :, 40] = sel[:, :, 10]
+    up[:, :, 100] = sel[:, :, 10] + 1e-3
+    # (2) up points ON selected points: finite output, that point carries (almost) all of the weight
+    up[:, :, :M] = sel
+    outs, idx, dist, nn_w = _interp_all(up, sel, feat)
+    assert torch.equal(outs[0], outs[1]) and torch.equal(outs[0], outs[2])
+    assert bool(torch.isfinite(outs[0]).all())
+    idx, nn_w = idx.cpu(), nn_w.cpu()
+    own = torch.arange(M).view(1, M, 1)
+    share = (nn_w[:, :M] * (idx[:, :M] == own)).sum(-1)                          # weight of the coincident point
+    for i in (10, 40):                                                            # (10 and 40 coincide)
+        share[:, i] = (nn_w[:, i] * ((idx[:, i] == 10) | (idx[:, i] == 40))).sum(-1)
+    print(f"coincident points: min weight share {float(share.min()):.6f}")
+    assert float(share.min()) >= 0.99
+    assert idx[0, 100, :2].tolist() == [10, 40] and float(dist[0, 100, 0]) == float(dist[0, 100, 1])
+    assert idx[0, 10, :2].tolist() == [10, 40] and idx[0, 40, :2].tolist() == [10, 40]
+    # fewer than three selected points: refused by all three
+    for fn in (lambda: ops.interpolate3(cu(up), cu(sel[..., :2]), cu(feat[..., :2])),
+               lambda: ops.interpolate3_rows(cu(up), cu(sel[..., :2]), cu(feat[..., :2].transpose(1, 2).contiguous()),
+                                             torch.empty(B, N, C, device=DEV)),
+               lambda: ops.interpolate3_search(cu(up), cu(sel[..., :2]))):
+        with pytest.raises(ValueError, match="at least 3"):
+            fn()
+
+
+# ---------------------------------------------------------------- dynamic bin boundaries, bit for bit
+
+
+def _aten_boundary_update(old, total, world, num_bins, momentum):
+    """utils/ops.py:198-233 as the reference states it (the oracle's update_sampling_score_bin_boundary after the
+    all_reduce), evaluated by ATen on whatever device `total` lives on"""
+    cut = total / world
+    if old is not None:
+        upper, lower = old[0].clone(), old[1].clone()
+        cut = upper[0, 0, 0, 1:] * momentum + (1 - momentum) * cut
+        upper[0, 0, 0, 1:] = cut
+        lower[0, 0, 0, :-1] = cut
+        return [upper, lower]
+    inf = torch.full((1,), float("inf"), device=total.device)
+    return [torch.cat([inf, cut]).reshape(1, 1, 1, num_bins), torch.cat([cut, -inf]).reshape(1, 1, 1, num_bins)]
+
+
+@pytest.mark.parametrize("nb", [2, 4, 6, 8])
+def test_boundary_update_bit_exact_vs_aten_on_the_gpu(nb):
+    """ops._quantile_pick + ops._boundary_ema (csrc/sampler.cu) against the reference's statement of utils/ops.py:182-233
+    run by ATen on the same GPU (the reference trains there), torch.equal: every rank count the bench shards over, fresh
+    pairs and EMA steps, two momentum factors, cloud sizes the bin count does not divide.  The ranks' local quantiles are
+    summed once and handed to both sides, as torch.distributed.all_reduce hands one sum to every rank."""
+    g = torch.Generator().manual_seed(nb)
+    cpu_diff = 0
+    for world in (1, 2, 3, 6, 8):
+        for n in (nb * 97 + 1, 1001, 2048 * 3 + nb - 1):
+            if n % nb == 0:
+                continue
+            for momentum in (0.99, 0.9):
+                state_native = state_aten = state_cpu = None
+                for step in range(3):                                          # fresh pair, then two EMA steps
+                    zs = [cu(torch.randn(n, generator=g) * (1 + step)) for _ in range(world)]
+                    ranked = [torch.sort(z, descending=True)[0] for z in zs]
+                    pos = (torch.arange(1, nb) / nb * n).int().long()         # utils/ops.py:182-189
+                    picks = [ops._quantile_pick(r, nb) for r in ranked]
+                    for p, r in zip(picks, ranked):
+                        assert torch.equal(p, r[pos.to(DEV)])
+                    total = picks[0].clone()
+                    for p in picks[1:]:
+                        total += p
+                    state_native = ops._boundary_ema(total, world, state_native, nb, momentum)
+                    state_aten = _aten_boundary_update(state_aten, total, world, nb, momentum)
+                    for a, b in zip(state_native, state_aten):
+                        assert torch.equal(a, b), (world, n, momentum, step, (a - b)[torch.isfinite(b)].abs().max().item())
+                    state_cpu = _aten_boundary_update(state_cpu, total.cpu(), world, nb, momentum)
+                    cpu_diff += sum(int((a.cpu() != b).sum()) for a, b in zip(state_aten, state_cpu))
+                    state_cpu = [t.cpu() for t in state_aten]                  # keep the CPU chain on the GPU's inputs
+    # ATen on the CPU divides by world; on CUDA it multiplies by the fp32 reciprocal: the CPU statement that stands in for
+    # the kernels in tests/test_distributed_cpu.py differs in the last bits of some boundaries (measured: 8 / 36 / 54 / 62
+    # values for nb = 2 / 4 / 6 / 8 over this sweep)
+    print(f"nb={nb}: CPU vs CUDA ATen statement: {cpu_diff} differing boundary values")

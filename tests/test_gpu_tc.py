@@ -172,18 +172,28 @@ def test_linear_pool_matches_fp64(case):
     assert torch.equal(mx, mx2) and torch.equal(mean, mean2)
 
 
-@pytest.mark.parametrize("case", [(2, 256, 128, 640), (3, 128, 64, 100), (2, 512, 1024, 128)], ids=lambda c: f"B{c[0]}_R{c[1]}_K{c[2]}_N{c[3]}")
+@pytest.mark.parametrize("case", [(2, 256, 128, 640), (3, 128, 64, 100), (2, 512, 1024, 128), (2, 256, 4096, 128), (1, 128, 4100, 64)],
+                         ids=lambda c: f"B{c[0]}_R{c[1]}_K{c[2]}_N{c[3]}")
 def test_cloud_matmul_matches_fp64(case):
-    """samble_cloud_matmul: per-cloud weights, and the softmax-row epilogue with known row statistics."""
+    """samble_cloud_matmul: per-cloud weights, and the softmax-row epilogue with known row statistics.  K = 4096 is the
+    longest contraction it takes (DownSampleToken's attention rows x V at N = 4096 keys, with the token share as the
+    residual); one key more is refused."""
     from samble_b200 import ops
 
     B, R, K, Nout = case
     g = torch.Generator().manual_seed(B + R + K)
     x = torch.randn(B, R, K, generator=g)
     w = torch.randn(B, Nout, K, generator=g) / K ** 0.5
+    if K > 4096:
+        with pytest.raises(ValueError, match="too large"):
+            ops.cloud_matmul(x.cuda(), w.cuda())
+        return
     ref = torch.matmul(x.double(), w.double().transpose(1, 2))
     y = ops.cloud_matmul(x.cuda(), w.cuda())
     assert (y.double().cpu() - ref).abs().max().item() < 2e-5 * max(1.0, ref.abs().max().item())
+    res = torch.randn(B, R, Nout, generator=g)
+    y_res = ops.cloud_matmul(x.cuda(), w.cuda(), residual=res.cuda())
+    assert (y_res.double().cpu() - ref - res.double()).abs().max().item() < 2e-5 * max(1.0, (ref + res.double()).abs().max().item())
     div = 3.0
     logits = ref / div
     rmax = logits.max(dim=-1)[0]
@@ -256,15 +266,18 @@ def test_xgemm_amax_feeds_the_next_slicing():
     assert float((rec == q.double()).double().mean()) > 0.95
 
 
-@pytest.mark.parametrize("B,N,nb,sharp", [(2, 2048, 4, 4.0), (1, 1000, 6, 8.0), (2, 512, 4, 1.0)])
-def test_ds_row_stats_exact_vs_fp64(B, N, nb, sharp):
+ROW_STATS_CASES = [(2, 2048, 4, 4.0, 128), (1, 1000, 6, 8.0, 128), (2, 512, 4, 1.0, 128), (2, 1000, 8, 4.0, 64)]
+
+
+@pytest.mark.parametrize("B,N,nb,sharp,D", ROW_STATS_CASES,
+                         ids=["-".join(map(str, c[:4])) + ("" if c[4] == 128 else f"-D{c[4]}") for c in ROW_STATS_CASES])
+def test_ds_row_stats_exact_vs_fp64(B, N, nb, sharp, D):
     """logsumexp of q [k | k_tok]^T / sqrt(D) from the exact GEMM: error of one fp32 rounding of the logit, not of a
     tensor-core accumulation chain."""
     import math
 
     from samble_b200 import ops
 
-    D = 128
     g = torch.Generator().manual_seed(N + nb)
     q = (torch.randn(B, N, D, generator=g) * sharp).cuda()
     k = torch.randn(B, N, D, generator=g).cuda()
