@@ -27,7 +27,12 @@ def wants_grad(*tensors) -> bool:
 
 
 def _bits(idx: Tensor) -> int:
-    return 64 if idx.dtype == torch.int64 else 32
+    """Index width for the C ABI; any dtype other than int32 / int64 would be read as garbage, so it is refused."""
+    if idx.dtype == torch.int64:
+        return 64
+    if idx.dtype == torch.int32:
+        return 32
+    raise TypeError(f"index tensor must be int32 or int64, got {idx.dtype}")
 
 
 def _scatter_rows(grad_rows: Tensor, idx: Tensor, N: int) -> Tensor:

@@ -30,12 +30,26 @@ def _f32(t: Tensor, name: str) -> Tensor:
     return t
 
 
-def _idx_bits(idx: Tensor) -> int:
-    if idx.dtype == torch.int64:
-        return 64
-    if idx.dtype == torch.int32:
-        return 32
-    raise TypeError(f"index tensor must be int32 or int64, got {idx.dtype}")
+_idx_bits = AG._bits
+
+
+def _rows(t: Tensor, name: str) -> Tensor:
+    """t (B,N,W) float32 as rows a kernel addresses with one row pitch t.stride(1): unit inner stride, a batch pitch of
+    N rows, 16-byte aligned rows.  A contiguous tensor or an aligned column slice of a wider row-major buffer passes as it
+    is; anything else is copied."""
+    _f32(t, name)
+    if (t.stride(2) != 1 or t.stride(0) != t.shape[1] * t.stride(1) or t.stride(1) % 4 != 0
+            or t.data_ptr() % 16 != 0):
+        t = t.clone(memory_format=torch.contiguous_format)       # (fresh storage: aligned even if t was contiguous)
+    return t
+
+
+def _neighbour_idx(idx: Tensor, B: int, N: int) -> Tensor:
+    """idx (B,N,K) int32 / int64 as the contiguous array the kernels index."""
+    _idx_bits(idx)
+    if idx.dim() != 3 or tuple(idx.shape[:2]) != (B, N):
+        raise RuntimeError(f"neighbour indices must be ({B},{N},K), got {tuple(idx.shape)}")
+    return idx.contiguous()
 
 
 # ------------------------------------------------------------------ kNN
@@ -499,7 +513,9 @@ def edge_mlp_max(pr: Tensor, idx: Tensor, w2: Tensor, b2: Tensor, out_rows: Opti
     The result is stored point-major -- in `out_rows` (B,N,C2), which may be a column slice of a wider row-major buffer, or
     in fresh storage -- and handed back in the reference's (B,C2,N) shape as a view of it (ops.rows_of is then free)."""
     dev = L.need_cuda(pr, idx, w2, b2, out_rows)
+    pr = _rows(pr, "pr")
     B, N, two_c1 = pr.shape
+    idx = _neighbour_idx(idx, B, N)
     C1, C2, K = two_c1 // 2, w2.shape[0], idx.shape[-1]
     w2, b2 = w2.contiguous(), b2.contiguous()
     if out_rows is None:
@@ -517,12 +533,15 @@ def n2p_attend(qkv: Tensor, idx: Tensor, heads: int, residual: Optional[Tensor] 
     Core of models/attention.py:165-185,207-250 with the k/v convolutions hoisted (attention.cu).
     With residual (B,N,C) / scale,shift (C,): returns (residual + attention) * scale + shift (folded bn1, :187)."""
     dev = L.need_cuda(qkv, idx, residual, scale, shift)
+    _f32(qkv, "qkv")
     if AG.wants_grad(qkv, residual, scale, shift):
         y = AG.N2PAttend.apply(qkv, idx, heads)
         if residual is not None:
             y = y + residual
         return y * scale + shift if scale is not None else y
+    qkv = _rows(qkv, "qkv")
     B, N, C3 = qkv.shape
+    idx = _neighbour_idx(idx, B, N)
     Cc = C3 // 3
     K = idx.shape[-1]
     out = torch.empty(B, N, Cc, dtype=torch.float32, device=dev)
@@ -531,7 +550,7 @@ def n2p_attend(qkv: Tensor, idx: Tensor, heads: int, residual: Optional[Tensor] 
         residual = residual.contiguous()
     if scale is not None:
         scale, shift = scale.contiguous(), shift.contiguous()
-    L.check(L.lib().samble_n2p_attend(L.ptr(q), L.ptr(k), L.ptr(v), C3, L.ptr(idx), _idx_bits(idx), B, N, Cc, K, heads,
+    L.check(L.lib().samble_n2p_attend(L.ptr(q), L.ptr(k), L.ptr(v), qkv.stride(1), L.ptr(idx), _idx_bits(idx), B, N, Cc, K, heads,
                                       L.ptr(residual), Cc, L.ptr(scale), L.ptr(shift), L.ptr(out), Cc, L.stream()),
             "samble_n2p_attend")
     return out
@@ -688,8 +707,11 @@ def ds_row_stats(q: Tensor, k: Tensor, k_tok: Tensor, k_split=None):
 
 def ds_edge_score(q: Tensor, k: Tensor, rowmax: Tensor, rowsum: Tensor, idx: Tensor) -> Tensor:
     """sparse_col_sqr point score (B,N) from the kNN edges only.  models/downsample.py:300-344."""
-    dev = L.need_cuda(q, k, idx)
+    dev = L.need_cuda(q, k, rowmax, rowsum, idx)
+    q, k = _rows(q, "q"), _rows(k, "k")
     B, N, D = q.shape
+    idx = _neighbour_idx(idx, B, N)
+    rowmax, rowsum = _f32(rowmax, "rowmax").contiguous(), _f32(rowsum, "rowsum").contiguous()
     K = idx.shape[-1]
     lib = L.lib()
     score = torch.empty(B, N, dtype=torch.float32, device=dev)

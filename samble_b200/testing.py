@@ -7,6 +7,7 @@ the oracle and the native ops when called: they serve the GPU tests only.
 """
 from __future__ import annotations
 
+import math
 import zlib
 from typing import Dict, Tuple
 
@@ -279,6 +280,22 @@ def judge_against_reference_scores(ds, idx: Tensor, x_ds: Tensor, ref_score: Ten
     ok = ((x_ds.cpu().double() - ref_x_ds.double()).abs() <= 2e-4 + 2e-4 * ref_x_ds.double().abs())       # (B,C,M)
     assert bool(ok[same.expand_as(ok)].all()), "x_ds rows of identically chosen points differ"
     return rep
+
+
+def n2p_attend_literal(qkv: Tensor, idx: Tensor, heads: int) -> Tensor:
+    """The reference's Neighbor2Point attention core in its own gathered-difference form (models/attention.py:165-185,
+    207-250): k_ij = k_j - k_i, v_ij = v_j - v_i, out_i = sum_j softmax_j(q_i . k_ij / sqrt(d)) v_ij per head, on the
+    hoisted projections qkv (B,N,3C) = [q|k|v] and idx (B,N,K).  Runs in qkv's dtype and device and is differentiable, so
+    fp64 autograd of it is the gradient reference of ops.n2p_attend."""
+    B, N, C3 = qkv.shape
+    C, K = C3 // 3, idx.shape[-1]
+    D = C // heads
+    q, k, v = qkv[..., :C], qkv[..., C:2 * C], qkv[..., 2 * C:]
+    flat = idx.long().reshape(B, -1, 1).expand(-1, -1, C)
+    kd = (torch.gather(k, 1, flat).view(B, N, K, C) - k[:, :, None, :]).view(B, N, K, heads, D)
+    vd = (torch.gather(v, 1, flat).view(B, N, K, C) - v[:, :, None, :]).view(B, N, K, heads, D)
+    att = torch.softmax(torch.einsum("bnhd,bnkhd->bnhk", q.reshape(B, N, heads, D), kd) / math.sqrt(D), dim=-1)
+    return torch.einsum("bnhk,bnkhd->bnhd", att, vd).reshape(B, N, C)
 
 
 def max_abs_rel(x: Tensor, ref: Tensor) -> Tuple[float, float]:

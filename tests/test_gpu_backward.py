@@ -6,7 +6,6 @@ model against the CPU oracle's autograd with the discrete decisions forced (orac
 (running-statistics BatchNorm) and in train mode (batch statistics).
 
 Tolerance: |g - g_ref|_inf <= 1e-4 * |g_ref|_inf per tensor (fp32 sums in another order; atomics)."""
-import math
 
 import pytest
 import torch
@@ -15,7 +14,7 @@ from torch import nn
 from oracle import harness
 from samble_b200 import blocks, models, ops
 from samble_b200.config import cls_config, seg_config
-from samble_b200.testing import fill_state_dict_, synthetic_clouds, synthetic_features
+from samble_b200.testing import fill_state_dict_, n2p_attend_literal, synthetic_clouds, synthetic_features
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -107,14 +106,8 @@ def test_n2p_attend_backward_matches_the_literal_form(B, N, C, K, H):
     qkv = torch.randn(B, N, 3 * C, generator=g)
     idx = torch.stack([torch.stack([torch.randperm(N, generator=g)[:K] for _ in range(N)]) for _ in range(B)])     # (B,N,K)
     probe = torch.randn(B, N, C, generator=g)
-    D = C // H
     r = qkv.double().requires_grad_(True)
-    q, k, v = r[..., :C], r[..., C:2 * C], r[..., 2 * C:]
-    gat = lambda t: torch.gather(t, 1, idx.reshape(B, -1, 1).expand(-1, -1, C)).view(B, N, K, C)
-    kd = (gat(k) - k[:, :, None, :]).view(B, N, K, H, D)
-    vd = (gat(v) - v[:, :, None, :]).view(B, N, K, H, D)
-    att = torch.softmax(torch.einsum("bnhd,bnkhd->bnhk", q.view(B, N, H, D), kd) / math.sqrt(D), dim=-1)
-    ref = torch.einsum("bnhk,bnkhd->bnhd", att, vd).reshape(B, N, C)
+    ref = n2p_attend_literal(r, idx, H)
     (g_ref,) = torch.autograd.grad((ref * probe.double()).sum(), r, retain_graph=True)
     for dt in (torch.int32, torch.int64):
         rc = qkv.to(DEV).requires_grad_(True)
