@@ -263,6 +263,38 @@ int samble_n2p_attend_backward(const float* q, const float* k, const float* v, l
                                int B, int N, int C, int K, int heads, const float* grad_out, long long ld_go,
                                float* grad_q, float* grad_k, float* grad_v, long long ld_g, samble_stream_t stream);
 
+/* ---- ordered backward scatters (csrc/backward_ordered.cu): the same gradients as the atomic entry points above with a
+ * defined summation order, so they are bitwise reproducible (what the Python layer runs under
+ * torch.use_deterministic_algorithms(True)).  For cloud b, edge e in [0,R) has target t_e = idx[b,e]; L_j lists the edges
+ * with target j in ascending e.  Each output element is the fp32 left fold, every product and sum rounded on its own:
+ *   acc = 0;  for e in L_j: acc = acc + term_e;   out[b,j,c] = acc  (or acc - sub[b,j,c])
+ *   term_e = x[b, e/src_div, c]   or, with a weight,   w[b,e,c/(C/heads)] * x[b, e/src_div, c].
+ * Entries of idx outside [0,N) contribute nothing.
+ *
+ * samble_reverse_index: idx (B,R) int32/int64 -> offsets (B,N+1) int32 and edges (B,R) int32, the edges of target j at
+ * edges[b, offsets[b,j] .. offsets[b,j+1]) in ascending e (a stable counting sort, one CTA per cloud); slots past
+ * offsets[b,N] (out-of-range entries) are set to -1.  ws: samble_reverse_index_workspace_bytes(B, N). */
+size_t samble_reverse_index_workspace_bytes(int B, int N);
+int samble_reverse_index(const void* idx, int idx_bits, int B, int N, int R, int* offsets, int* edges, void* ws, size_t ws_bytes,
+                         samble_stream_t stream);
+/* samble_scatter_rows_ordered: the fold above, WRITING out (every element of out (B,N,C) is written; nothing needs zeroing).
+ * x element (b, row, c) at x[b*x_batch + row*x_row + c*x_ch], out likewise with out_*: row-major and channel-major layouts
+ * and column slices of wider buffers are all strides.  w (B,R,heads) contiguous or NULL; sub (B,N,C) with unit channel
+ * stride at sub[b*sub_batch + j*sub_row + c], or NULL.  One warp per target row: its time is proportional to the largest
+ * in-degree, so a hub target that every edge lists runs as one serial fold. */
+int samble_scatter_rows_ordered(const float* x, long long x_batch, long long x_row, long long x_ch, int src_div,
+                                const float* w, int heads, const int* offsets, const int* edges, const float* sub,
+                                long long sub_batch, long long sub_row, int B, int N, int R, int C, float* out,
+                                long long out_batch, long long out_row, long long out_ch, samble_stream_t stream);
+/* samble_n2p_attend_backward_edges: samble_n2p_attend_backward's per-edge pass without its scatter.  Same arguments and limits;
+ * writes grad_q (ld_g) and, per edge e = n*K + slot and head h, p[(b*N*K + e)*heads + h] = p_ij and ds[...] = ds_ij, the very
+ * fp32 values the atomic kernel multiplies into its atomics.  Then, with the reverse index of idx (R = N*K):
+ *   grad_k = samble_scatter_rows_ordered(x = q,        src_div = K, w = ds)
+ *   grad_v = samble_scatter_rows_ordered(x = grad_out, src_div = K, w = p, sub = grad_out). */
+int samble_n2p_attend_backward_edges(const float* q, const float* k, const float* v, long long ld, const void* idx, int idx_bits,
+                                     int B, int N, int C, int K, int heads, const float* grad_out, long long ld_go,
+                                     float* grad_q, long long ld_g, float* p, float* ds, samble_stream_t stream);
+
 /* --------------------------------------------------- DownSampleToken scoring ----
  * models/downsample.py:124-153: energy = q @ [k | k_tok] / sqrt(D), row softmax over
  * N+nb columns.  The N x (N+nb) map is never written: this pass leaves per-row

@@ -42,7 +42,11 @@ PROTOTYPES: Dict[str, Tuple[object, tuple]] = {
     "samble_index_points_backward": (_i, (_p, _p, _i, _i, _i, _i, _i, _p, _p)),
     "samble_gather_by_idx_backward": (_i, (_p, _p, _i, _i, _i, _i, _i, _p, _p)),
     "samble_n2p_attend_backward": (_i, (_p, _p, _p, _ll, _p, _i, _i, _i, _i, _i, _i, _p, _ll, _p, _p, _p, _ll, _p)),
-    "samble_transpose": (_i, (_p, _ll, _ll, _i, _i, _i, _p, _p)),
+    "samble_reverse_index_workspace_bytes": (_sz, (_i, _i)),
+    "samble_reverse_index": (_i, (_p, _i, _i, _i, _i, _p, _p, _p, _sz, _p)),
+    "samble_scatter_rows_ordered": (_i, (_p, _ll, _ll, _ll, _i, _p, _i, _p, _p, _p, _ll, _ll, _i, _i, _i, _i, _p, _ll, _ll, _ll, _p)),
+    "samble_n2p_attend_backward_edges": (_i, (_p, _p, _p, _ll, _p, _i, _i, _i, _i, _i, _i, _p, _ll, _p, _ll, _p, _p, _p)),
+    "samble_transpose": (_i,(_p, _ll, _ll, _i, _i, _i, _p, _p)),
     "samble_neighbor_mask": (_i, (_p, _i, _i, _i, _i, _p, _p)),
     "samble_split_tf32": (_i, (_p, _p, _ll, _p)),
     "samble_ds_row_stats_fast_workspace_bytes": (_sz, (_i, _i)),

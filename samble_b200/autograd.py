@@ -10,6 +10,11 @@ What is native here: the gathers and their scatter-add backward, the Neighbor2Po
 (nothing of size N*K*C is saved or formed in either direction: the forward saves the (B,N,3C) projections and the
 indices, the backward recomputes the probabilities), and the distance gradient in at::_euclidean_dist_backward's form
 evaluated only on the k selected pairs.  Dense layers (1x1 convolutions, BatchNorm with batch statistics) stay ATen.
+
+The scatters of these backward passes add their terms with fp32 atomics (csrc/backward.cu), so the last bits of a
+gradient change from run to run.  While torch.use_deterministic_algorithms(True) is in force -- the switch ATen's own
+gather backward honours -- they take the ordered kernels of csrc/backward_ordered.cu instead: a reverse neighbour index
+built once per backward call, then a fold of each target's terms in ascending edge order, bitwise reproducible.
 """
 from __future__ import annotations
 
@@ -35,9 +40,63 @@ def _bits(idx: Tensor) -> int:
     raise TypeError(f"index tensor must be int32 or int64, got {idx.dtype}")
 
 
+def deterministic() -> bool:
+    """True while torch.use_deterministic_algorithms(True) is in force (with or without warn_only): the backward scatters
+    then take the ordered kernels of csrc/backward_ordered.cu instead of the fp32 atomics of csrc/backward.cu."""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def reverse_index(idx: Tensor, N: int):
+    """idx (B, ...) int32 / int64, flattened per cloud to (B,R) -> (offsets (B,N+1) int32, edges (B,R) int32): the edges of
+    target j are edges[b, offsets[b,j]:offsets[b,j+1]] in ascending order; entries outside [0,N) are left out."""
+    idx = idx.contiguous()
+    B = idx.shape[0]
+    R = idx[0].numel()
+    dev = idx.device
+    offsets = torch.empty(B, N + 1, dtype=torch.int32, device=dev)
+    edges = torch.empty(B, R, dtype=torch.int32, device=dev)
+    lib = L.lib()
+    ws = L.workspace(lib.samble_reverse_index_workspace_bytes(B, N), dev)
+    L.check(lib.samble_reverse_index(L.ptr(idx), _bits(idx), B, N, R, L.ptr(offsets), L.ptr(edges), L.ptr(ws), ws.numel(),
+                                     L.stream()), "samble_reverse_index")
+    return offsets, edges
+
+
+def scatter_rows_ordered(x: Tensor, offsets: Tensor, edges: Tensor, *, channel_major: bool = False, weight: Tensor = None,
+                         src_div: int = 1, sub: Tensor = None, out: Tensor = None) -> Tensor:
+    """The ordered scatter: out[b, j, c] = fold over the edges e of target j (ascending) of weight[b, e, h(c)] * x[b, e // src_div, c]
+    (weight None: x alone), minus sub[b, j, c] if given.  x (B,S,C) rows, or (B,C,S) when channel_major, any strides;
+    weight (B,R,heads); sub (B,N,C) with unit channel stride; out (B,N,C) (or (B,C,N)) is written, allocated if None."""
+    B, N = offsets.shape[0], offsets.shape[1] - 1
+    R = edges.shape[1]
+    if channel_major:
+        C = x.shape[1]
+        xs = (x.stride(0), x.stride(2), x.stride(1))
+    else:
+        C = x.shape[2]
+        xs = (x.stride(0), x.stride(1), x.stride(2))
+    if out is None:
+        out = torch.empty((B, C, N) if channel_major else (B, N, C), dtype=torch.float32, device=x.device)
+    os_ = (out.stride(0), out.stride(2), out.stride(1)) if channel_major else (out.stride(0), out.stride(1), out.stride(2))
+    heads = 1
+    if weight is not None:
+        weight = weight.contiguous()
+        heads = weight.shape[-1]
+    if sub is not None and sub.stride(2) != 1:
+        sub = sub.contiguous()
+    sb = (sub.stride(0), sub.stride(1)) if sub is not None else (0, 0)
+    L.check(L.lib().samble_scatter_rows_ordered(L.ptr(x), *xs, src_div, L.ptr(weight), heads, L.ptr(offsets), L.ptr(edges),
+                                                L.ptr(sub), *sb, B, N, R, C, L.ptr(out), *os_, L.stream()),
+            "samble_scatter_rows_ordered")
+    return out
+
+
 def _scatter_rows(grad_rows: Tensor, idx: Tensor, N: int) -> Tensor:
     """grad_rows (B,R,C) contiguous, idx (B,R) -> (B,N,C) with out[b, idx[b,r]] += grad_rows[b,r]."""
     B, R, C = grad_rows.shape
+    if deterministic():
+        offsets, edges = reverse_index(idx, N)
+        return scatter_rows_ordered(grad_rows, offsets, edges)
     out = torch.zeros(B, N, C, dtype=torch.float32, device=grad_rows.device)
     L.check(L.lib().samble_index_points_backward(L.ptr(grad_rows), L.ptr(idx), _bits(idx), B, N, C, R, L.ptr(out), L.stream()),
             "samble_index_points_backward")
@@ -120,6 +179,9 @@ class GatherByIdx(Function):
         (idx,) = ctx.saved_tensors
         g = g.contiguous()
         B, C, M = g.shape
+        if deterministic():
+            offsets, edges = reverse_index(idx.view(B, M), ctx.n)
+            return scatter_rows_ordered(g, offsets, edges, channel_major=True), None
         out = torch.zeros(B, C, ctx.n, dtype=torch.float32, device=g.device)
         L.check(L.lib().samble_gather_by_idx_backward(L.ptr(g), L.ptr(idx), _bits(idx), B, C, ctx.n, M, L.ptr(out), L.stream()),
                 "samble_gather_by_idx_backward")
@@ -155,12 +217,45 @@ class N2PAttend(Function):
         g = g.contiguous()
         B, N, C3 = qkv.shape
         C, K = C3 // 3, idx.shape[-1]
+        if deterministic():
+            return n2p_attend_backward_ordered(qkv, idx, ctx.heads, g), None, None
         gqkv = torch.zeros_like(qkv)
         q, k, v = (Ct.c_void_p(qkv.data_ptr() + 4 * C * i) for i in range(3))
         gq, gk, gv = (Ct.c_void_p(gqkv.data_ptr() + 4 * C * i) for i in range(3))
         L.check(L.lib().samble_n2p_attend_backward(q, k, v, C3, L.ptr(idx), _bits(idx), B, N, C, K, ctx.heads, L.ptr(g), C,
                                                    gq, gk, gv, C3, L.stream()), "samble_n2p_attend_backward")
         return gqkv, None, None
+
+
+def n2p_attend_backward_edges(qkv: Tensor, idx: Tensor, heads: int, g: Tensor, grad_q: Tensor = None):
+    """The per-edge pass of the ordered N2P backward: qkv (B,N,3C) contiguous, idx (B,N,K), g (B,N,C) contiguous ->
+    (grad_q, p, ds): grad_q (B,N,C) (or written into the given (B,N,*) view with unit inner stride), p / ds (B,N,K,heads)."""
+    import ctypes as Ct
+
+    B, N, C3 = qkv.shape
+    C, K = C3 // 3, idx.shape[-1]
+    if grad_q is None:
+        grad_q = torch.empty(B, N, C, dtype=torch.float32, device=qkv.device)
+    p = torch.empty(B, N, K, heads, dtype=torch.float32, device=qkv.device)
+    ds = torch.empty_like(p)
+    q, k, v = (Ct.c_void_p(qkv.data_ptr() + 4 * C * i) for i in range(3))
+    L.check(L.lib().samble_n2p_attend_backward_edges(q, k, v, C3, L.ptr(idx), _bits(idx), B, N, C, K, heads, L.ptr(g), C,
+                                                     L.ptr(grad_q), grad_q.stride(1), L.ptr(p), L.ptr(ds), L.stream()),
+            "samble_n2p_attend_backward_edges")
+    return grad_q, p, ds
+
+
+def n2p_attend_backward_ordered(qkv: Tensor, idx: Tensor, heads: int, g: Tensor) -> Tensor:
+    """N2PAttend's gradient w.r.t. qkv without atomics: the edge pass, then dk_j = fold of ds_ij q_i and
+    dv_j = (fold of p_ij g_i) - g_j over the edges i -> j in ascending i*K + slot."""
+    B, N, C3 = qkv.shape
+    C, K = C3 // 3, idx.shape[-1]
+    gqkv = torch.empty_like(qkv)
+    _, p, ds = n2p_attend_backward_edges(qkv, idx, heads, g, grad_q=gqkv[..., :C])
+    offsets, edges = reverse_index(idx.view(B, N * K), N)
+    scatter_rows_ordered(qkv[..., :C], offsets, edges, weight=ds.view(B, N * K, heads), src_div=K, out=gqkv[..., C:2 * C])
+    scatter_rows_ordered(g, offsets, edges, weight=p.view(B, N * K, heads), src_div=K, sub=g, out=gqkv[..., 2 * C:])
+    return gqkv
 
 
 class PairDistance(Function):

@@ -6,7 +6,9 @@
 // forward kernels use: the (B,C,N,K) grouped tensors of the reference's attention never exist in either direction.
 //
 // Accumulation uses fp32 atomics (RED.ADD): summation order, hence the last bits of a gradient, varies run to run,
-// as it does in ATen's own gather backward (index_add / scatter_add on CUDA).
+// as it does in ATen's own gather backward (index_add / scatter_add on CUDA) while torch.use_deterministic_algorithms is
+// off.  With it on, ATen switches to ordered algorithms and so does this library: samble_b200/autograd.py then runs the
+// atomic-free kernels of backward_ordered.cu instead, which add the same terms in a defined order.
 #include "common.cuh"
 
 namespace samble {

@@ -231,6 +231,46 @@ def gather_by_idx(pcd: Tensor, idx: Tensor) -> Tensor:
     return out
 
 
+# ------------------------------------------------------------------ ordered backward scatters
+#
+# The kernels the differentiable path runs under torch.use_deterministic_algorithms(True) (autograd.py), exposed one by
+# one so their order contract can be checked directly.
+
+
+def reverse_index(idx: Tensor, N: int) -> Tuple[Tensor, Tensor]:
+    """idx (B, ...) int32 / int64 over N targets -> (offsets (B,N+1) int32, edges (B,R) int32), R = idx[0].numel(): the
+    flat positions e with idx[b].flatten()[e] == j are edges[b, offsets[b,j]:offsets[b,j+1]], ascending.  Entries outside
+    [0,N) are left out (offsets[b,N] counts the rest; the slots after it hold -1)."""
+    L.need_cuda(idx)
+    _idx_bits(idx)
+    return AG.reverse_index(idx.reshape(idx.shape[0], -1), N)
+
+
+def scatter_rows_ordered(x: Tensor, offsets: Tensor, edges: Tensor, *, channel_major: bool = False,
+                         weight: Optional[Tensor] = None, src_div: int = 1, sub: Optional[Tensor] = None) -> Tensor:
+    """out[b,j,c] = sum over the edges e of target j, in ascending e, of weight[b,e,c // (C/heads)] * x[b, e // src_div, c]
+    (x alone without a weight) as an fp32 left fold, minus sub[b,j,c] if given.  x (B,S,C), or (B,C,S) with channel_major
+    (then the result is (B,C,N) too); weight (B,R,heads); sub (B,N,C)."""
+    L.need_cuda(x, offsets, edges, weight, sub)
+    _f32(x, "x")
+    for t, name in ((weight, "weight"), (sub, "sub")):
+        if t is not None:
+            _f32(t, name)
+    if offsets.dtype != torch.int32 or edges.dtype != torch.int32:
+        raise TypeError("offsets and edges must be int32 (ops.reverse_index)")
+    return AG.scatter_rows_ordered(x, offsets.contiguous(), edges.contiguous(), channel_major=channel_major, weight=weight,
+                                   src_div=src_div, sub=sub)
+
+
+def n2p_attend_backward_edges(qkv: Tensor, idx: Tensor, heads: int, grad_out: Tensor) -> Tuple[Tensor, Tensor, Tensor]:
+    """The per-edge pass of the ordered Neighbor2Point backward: qkv (B,N,3C) = [q|k|v], idx (B,N,K), grad_out (B,N,C) ->
+    (grad_q (B,N,C), p (B,N,K,heads), ds (B,N,K,heads)) with the atomic kernel's own fp32 values of p_ij and ds_ij."""
+    L.need_cuda(qkv, idx, grad_out)
+    qkv = _f32(qkv, "qkv").contiguous()
+    B, N = qkv.shape[:2]
+    return AG.n2p_attend_backward_edges(qkv, _neighbour_idx(idx, B, N), heads, _f32(grad_out, "grad_out").contiguous())
+
+
 # ------------------------------------------------------------------ fused block cores
 
 
