@@ -111,6 +111,21 @@ def knn_parity(idx: Tensor, ref_idx: Tensor, a: Tensor, b: Tensor, rel_band: flo
                 unexplained_rows=unexplained)
 
 
+def launched(fn):
+    """(fn(), {kernel name: launches}) over the native launches fn makes (the names of SAMBLE_LAUNCHED in csrc/)."""
+    from . import _lib as L
+
+    torch.cuda.synchronize()
+    L.profile_report()                                   # drop anything recorded earlier
+    L.profile(True)
+    try:
+        out = fn()
+        torch.cuda.synchronize()
+    finally:
+        L.profile(False)
+    return out, {name: n for name, (n, _) in L.profile_report().items()}
+
+
 def sampled_index_parity(idx: Tensor, ref_idx: Tensor, score: Tensor, k_per_bin: Tensor) -> dict:
     """Tie-aware sampler comparison.  idx/ref_idx (B,1,M) int64, score (B,1,N) is the
     REFERENCE score, k_per_bin (B,nb).  Indices must be equal except inside groups of

@@ -10,10 +10,10 @@ import pytest
 import torch
 
 from oracle import samble_oracle as O
-from samble_b200 import _lib as L
 from samble_b200 import blocks, ops
 from samble_b200.config import Cfg, _attention, _downsample
-from samble_b200.testing import amp_excusing_knn_ties, fill_state_dict_, judge_against_reference_scores, synthetic_features
+from samble_b200.testing import (amp_excusing_knn_ties, fill_state_dict_, judge_against_reference_scores, launched,
+                                 synthetic_features)
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
@@ -26,19 +26,6 @@ def cu(t):
 def close_frac(x, ref, atol=2e-4, rtol=2e-4):
     x, ref = x.detach().cpu().double(), ref.detach().cpu().double()
     return float(((x - ref).abs() <= atol + rtol * ref.abs()).double().mean())
-
-
-def launched(fn):
-    """(fn(), {kernel name: launches}) over the native launches fn makes (the names of SAMBLE_LAUNCHED in csrc/)."""
-    torch.cuda.synchronize()
-    L.profile_report()                                   # drop anything recorded earlier
-    L.profile(True)
-    try:
-        out = fn()
-        torch.cuda.synchronize()
-    finally:
-        L.profile(False)
-    return out, {name: n for name, (n, _) in L.profile_report().items()}
 
 
 def filled(block, seed, sharpen=1.0):
